@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200 Hades engine (driver contract).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload W]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload W] [--dump-outputs DIR]
 
 Workload (default `merkle4`, BASELINE.json configs[1]): one step = one batch of 2^20 independent
 `Hash::digest(Domain::Merkle4, 4 scalars)` per GPU = 2^20 width-5 Hades permutations per GPU, on
@@ -24,6 +24,9 @@ Other workloads (not the driver's headline; used for profiles/ and DESIGN.md num
   --workload sweep     Domain::Other, EVERY in_len 1..256 at 2^18 items (configs[4]); per-length table in `sweep`
                        (--sweep-lens 1,2,4 to subsample)
   --workload tree      the tree build alone (--log4-leaves k)                  --workload convert  wire-format kernel
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step computed as DIR/<name>.npy, so that two
+builds can be compared output for output on identical seeded inputs (see dump_outputs).
 """
 import argparse
 import json
@@ -42,6 +45,7 @@ LOG2_BATCH = 20
 BYTES_PER_PERM = 160          # Merkle4 digest: 4 x 32 B in + 32 B out (SURVEY.md 8d)
 SM_COUNT = 148
 TREE_LOG4 = {1: 11, 2: 12, 4: 13, 8: 14}
+DUMP_ROWS = 1 << 16           # items kept per dumped array (4 MiB for Merkle4 digests)
 
 
 def env_int(name, default):
@@ -130,6 +134,24 @@ def ncu_traffic():
     return None
 
 
+def dump_outputs(directory, arrays, rank, world):
+    """Writes each array (numpy or torch, first axis = items) as <directory>/<name>.npy in float64, one row per item.
+    Batches larger than DUMP_ROWS items keep a fixed seeded sample of DUMP_ROWS rows in item order.  Every 64-bit word
+    is split into its 32-bit halves, low half first, so that each value is exact in float64.  With more than one rank,
+    each rank writes <name>_rank<r>.npy."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    suffix = "" if world == 1 else "_rank%d" % rank
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if hasattr(a, "cpu") else np.asarray(a)
+        a = np.ascontiguousarray(a.reshape(a.shape[0], -1))
+        if a.shape[0] > DUMP_ROWS:
+            a = a[np.sort(np.random.default_rng(0xD0).choice(a.shape[0], DUMP_ROWS, replace=False))]
+        if a.dtype.itemsize == 8:
+            a = a.view(np.uint32)
+        np.save(os.path.join(directory, name + suffix + ".npy"), a.astype(np.float64))
+
+
 def workload_config(log2_batch, world):
     """`config` of the headline workload -- built by ONE function so that the GPU arm and the reference arm print the
     identical object (the driver compares them)."""
@@ -202,6 +224,8 @@ def run_reference_arm(args, rank, world, emit):
     for _ in range(args.warmup):
         arm.run(threads, per_step)
     dts = [arm.run(threads, per_step) for _ in range(args.steps)]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"digests": arm.out[:per_step]}, rank, 1)
     total = sum(dts)
     value = per_step * args.steps / total
     sample = "%d digests per step x %d steps, %d pthreads; hashing call timed alone (inputs/tag generated once, outside)" % (
@@ -375,9 +399,15 @@ def main():
     ap.add_argument("--sweep-lens", default="", help="sweep: comma-separated input lengths (default: every length 1..256)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-tree", action="store_true", help="merkle4: skip the tree block")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float64)")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 2 if args.workload == "sweep" else 40
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.workload == "tree" and args.impl == "b200":
+        ap.error("--dump-outputs is not supported with --workload tree")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank, world, local = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
 
@@ -452,12 +482,14 @@ def main():
             out = torch.empty((n, 1, 4), dtype=torch.int64, device="cuda")
         perms_per_step, bytes_per_step = n, n * BYTES_PER_PERM
         step = lambda i: pb.Hash.digest_batch(pb.Domain.Merkle4, ins[i % nbuf], engine=eng, out=out, async_=True)
+        outputs = lambda: {"digests": out}
         config = workload_config(args.log2_batch, world)
     elif args.workload == "permute":
         with torch.cuda.stream(stream):
             st = torch.from_numpy(random_limbs_fast(rng, (n, 5)).view(np.int64)).cuda()
         perms_per_step, bytes_per_step = n, n * 320
         step = lambda i: eng.permute_batch_inplace(st, async_=True)
+        outputs = lambda: {"states": st}
         workload, l2_note = "raw permute_batch of 2^%d x 5 states in place" % args.log2_batch, "160 MiB state array > L2"
     elif args.workload == "encrypt":
         with torch.cuda.stream(stream):
@@ -467,6 +499,7 @@ def main():
             cip = torch.empty((n, 3, 4), dtype=torch.int64, device="cuda")
         perms_per_step, bytes_per_step = 2 * n, n * 256
         step = lambda i: pb.encrypt_batch(msg, sec, non, engine=eng, out=cip, async_=True)
+        outputs = lambda: {"ciphertexts": cip}
         workload, l2_note = "encrypt_batch 2^%d messages, L=2 (benches/encrypt.rs:17)" % args.log2_batch, "256 MiB touched per step > L2"
     elif args.workload == "decrypt":
         with torch.cuda.stream(stream):
@@ -480,6 +513,7 @@ def main():
 
         def step(i):
             ok_holder["m"], ok_holder["ok"] = pb.decrypt_batch(cip, sec, non, engine=eng, async_=True)
+        outputs = lambda: {"messages": ok_holder["m"], "ok": ok_holder["ok"]}
         workload, l2_note = "decrypt_batch 2^%d ciphers, L=2 (benches/decrypt.rs:17)" % args.log2_batch, "257 MiB touched per step > L2"
     elif args.workload == "sweep":
         n = 1 << 18
@@ -502,6 +536,7 @@ def main():
                 e.record(stream)
                 evs.append(e)
             sweep_events.append(evs)
+        outputs = lambda: {"digests_in_len%d" % lens[-1]: out}        # `out` holds the step's last length
         workload = "sponge sweep Domain::Other, every in_len in [%d, %d] (%d lengths), batch 2^18 per length per GPU" % (
             min(lens), max(lens), len(lens))
         l2_note = "length L reads the first 2^18*L scalars of one %d MiB buffer (> L2 for L >= 16)" % (n * max(lens) * 32 >> 20)
@@ -513,6 +548,7 @@ def main():
         perms_per_step, bytes_per_step = n, n * 64       # "perms" here = scalars converted (no permutation)
         lib, ctx = eng._lib, eng._ctx
         step = lambda i: eng._check(lib.p252_scalars_to_bytes(ctx, sc.data_ptr(), n, ob.data_ptr(), 3))
+        outputs = lambda: {"bytes": ob}
         workload, l2_note = "to_bytes of 2^25 scalars (wire-format kernel, the one HBM-bound kernel); value = scalars/s", "1 GiB in + 1 GiB out per step"
     else:  # tree alone
         k = args.log4_leaves or TREE_LOG4.get(world, 12)
@@ -552,6 +588,8 @@ def main():
     barrier()
     clocks = sampler.stop()
     launches = eng.launch_count - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs(), rank, world)
     total_ms = ev[0].elapsed_time(ev[-1])
     per_step_ms = [ev[i].elapsed_time(ev[i + 1]) for i in range(args.steps)]
     if dist is not None:

@@ -39,6 +39,61 @@ def test_non_zero_ranks_of_the_reference_arm_exit_quietly():
 import pytest
 
 
+def _merkle4_oracle_words(data):
+    """Merkle4 digests of (n, 4, 4) limbs by the C oracle, as dump_outputs writes them: 32-bit words in float64."""
+    import numpy as np
+    sys.path.insert(0, os.path.join(ROOT, "oracle"))
+    sys.path.insert(0, ROOT)
+    import c_oracle
+    import hades_oracle as o
+    from poseidon252_b200.scalar import to_mont
+    tag = to_mont(o.hash_to_scalar(o.tag_input([o.Absorb(4), o.Squeeze(1)], o.Domain.Merkle4)))
+    return c_oracle.digest(tag, data, 4, 1).reshape(len(data), 4).view(np.uint32).astype(np.float64)
+
+
+def test_reference_arm_dump_outputs(tmp_path):
+    """--dump-outputs: the last step's digests, one float64 row of 8 exact 32-bit words per item, identical from run
+    to run and equal to the oracle on the arm's seeded inputs."""
+    import numpy as np
+    from poseidon252_b200.scalar import random_limbs_fast
+    dumps = []
+    for run in range(2):
+        d = tmp_path / str(run)
+        res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",
+                              "--warmup", "0", "--log2-batch", "10", "--dump-outputs", str(d)],
+                             capture_output=True, text=True, timeout=300, cwd=ROOT)
+        assert res.returncode == 0, res.stderr[-2000:]
+        assert sorted(os.listdir(d)) == ["digests.npy"]
+        dumps.append(np.load(d / "digests.npy"))
+    assert dumps[0].dtype == np.float64 and dumps[0].shape == (1 << 10, 8)
+    assert np.array_equal(dumps[0], dumps[1])
+    assert np.array_equal(dumps[0], _merkle4_oracle_words(random_limbs_fast(np.random.default_rng(123), (1 << 10, 4))))
+
+
+def test_steps_must_be_positive():
+    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                         capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert res.returncode != 0 and "--steps" in res.stderr
+
+
+@pytest.mark.gpu
+def test_gpu_arm_dump_outputs(tmp_path):
+    """--dump-outputs on the GPU arm: the digests of the last timed step (input buffer (steps - 1) % 4 of the seeded
+    rotation), bit-exact against the oracle."""
+    import numpy as np
+    from poseidon252_b200.scalar import random_limbs_fast
+    steps, log2 = 3, 12
+    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "3",
+                          "--log2-batch", str(log2), "--no-tree", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert res.returncode == 0, res.stderr[-3000:]
+    assert json.loads(res.stdout)["steps"] == steps
+    got = np.load(tmp_path / "digests.npy")
+    rng = np.random.default_rng(0xC10D)
+    ins = [random_limbs_fast(rng, (1 << log2, 4)) for _ in range(4)]
+    assert got.dtype == np.float64 and np.array_equal(got, _merkle4_oracle_words(ins[(steps - 1) % 4]))
+
+
 @pytest.mark.gpu
 def test_gpu_arm_line_small():
     """the GPU arm end to end on a reduced batch: one JSON line, contract keys, roofline / imad / e2e / tree blocks,

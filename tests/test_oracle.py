@@ -7,7 +7,7 @@ import pytest
 
 from conftest import hx, mont, unmont
 
-REF = "/root/reference"
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def test_reference_kats(oracle):
@@ -19,11 +19,11 @@ def test_reference_kats(oracle):
 
 def test_constants_match_reference_assets(oracle):
     """Constants regenerated from assets/HOWTO.md equal the reference's .bin files byte for byte
-    (only checkable where /root/reference exists; the GPU box does not have it)."""
-    if not os.path.isdir(REF):
-        pytest.skip("reference checkout not present on this machine")
-    assert oracle.arc_bin_bytes() == open(os.path.join(REF, "assets/arc.bin"), "rb").read()
-    assert oracle.mds_bin_bytes() == open(os.path.join(REF, "assets/mds.bin"), "rb").read()
+    (tests/golden/arc.bin and mds.bin are unmodified copies of dusk-poseidon's assets/arc.bin and assets/mds.bin)."""
+    with open(os.path.join(GOLDEN, "arc.bin"), "rb") as f:
+        assert oracle.arc_bin_bytes() == f.read()
+    with open(os.path.join(GOLDEN, "mds.bin"), "rb") as f:
+        assert oracle.mds_bin_bytes() == f.read()
 
 
 def test_round_constants_nonzero_and_roundtrip(oracle):
