@@ -213,6 +213,19 @@ int p252_merkle_verify_batch(p252_ctx* ctx, int arity, int depth, const p252_fr*
                              const p252_fr* paths, const p252_fr* root, size_t n, uint8_t* ok, size_t* n_failed,
                              int flags);
 
+/* Overwrite k leaves of a tree held as leaves + nodes (the p252_merkle_build layout; arity 2 or 4, n_leaves = arity^depth)
+ * and recompute exactly the internal nodes on their paths.  Afterwards leaves/nodes equal p252_merkle_build of the
+ * updated leaves, bit for bit; no other node is written.  leaf_idx / values: k entries, any order; an index may repeat,
+ * the LAST occurrence in the batch wins (as k sequential writes would).  leaf_idx lives in the same memory space as the
+ * other buffers.  An index >= n_leaves: HOST -> P252_ERR_INVALID_ARGUMENT before anything is written; DEVICE -> that
+ * entry is skipped, the others are applied, and *n_rejected (optional HOST pointer, as n_failed of p252_decrypt_batch)
+ * receives the number skipped.  k = 0 is a no-op that launches nothing.
+ * HOST buffers: only the groups on the dirty paths cross PCIe, and leaves/nodes are written only after all device work
+ * succeeded (a failed call leaves the tree untouched).  DEVICE buffers: the plan (sort, dedupe, dirty lists per level)
+ * runs on the device with no host synchronisation; a failed call may leave the tree partially updated. */
+int p252_merkle_update_batch(p252_ctx* ctx, int arity, p252_fr* leaves, size_t n_leaves, p252_fr* nodes,
+                             const uint64_t* leaf_idx, const p252_fr* values, size_t k, size_t* n_rejected, int flags);
+
 /* ---- multi-GPU tree build: one process per GPU, one NCCL all-gather per level ---------------- */
 #define P252_NCCL_UNIQUE_ID_BYTES 128
 /* rank 0 creates the id and ships it to the other ranks by any means (torch.distributed / MPI) */

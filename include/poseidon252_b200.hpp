@@ -251,6 +251,21 @@ inline std::vector<Opening> merkle_open_batch(int arity, const std::vector<Scala
     return out;
 }
 
+// Write values[j] to leaf leaf_idx[j] (the last occurrence of a repeated index wins) and rehash only the dirty paths,
+// in place: afterwards leaves / nodes equal merkle_build(arity, leaves).  An index outside the tree throws
+// Error{P252_ERR_INVALID_ARGUMENT} and leaves the tree untouched.
+inline void merkle_update_batch(int arity, std::vector<Scalar>& leaves, std::vector<Scalar>& nodes,
+                                const std::vector<uint64_t>& leaf_idx, const std::vector<Scalar>& values,
+                                Engine& e = Engine::default_engine()) {
+    size_t n_internal = 0;
+    check(p252_merkle_tree_nodes(arity, leaves.size(), &n_internal, nullptr));
+    if (nodes.size() != n_internal) throw Error(P252_ERR_INVALID_ARGUMENT, "node array does not match the leaf count");
+    if (leaf_idx.size() != values.size()) throw Error(P252_ERR_INVALID_ARGUMENT, "leaf_idx and values differ in length");
+    check(p252_merkle_update_batch(e.get(), arity, leaves.data(), leaves.size(), nodes.data(), leaf_idx.data(),
+                                   values.data(), values.size(), nullptr, P252_MEM_HOST),
+          e.get());
+}
+
 // n x Opening::verify with all openings in one launch: ok[i] != 0 iff paths[i] proves items[i] under root
 inline std::vector<uint8_t> merkle_verify_batch(int arity, int depth, const Scalar* items, const uint64_t* leaf_idx,
                                                 const Scalar* paths, const Scalar& root, size_t n,

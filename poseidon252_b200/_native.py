@@ -50,6 +50,8 @@ SIGNATURES = {
     "p252_merkle_open_batch": (c_int, [c_void_p, c_int, c_void_p, c_size_t, c_void_p, c_void_p, c_size_t, c_void_p, c_int]),
     "p252_merkle_verify_batch": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p,
                                          ctypes.POINTER(c_size_t), c_int]),
+    "p252_merkle_update_batch": (c_int, [c_void_p, c_int, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_size_t,
+                                         ctypes.POINTER(c_size_t), c_int]),
     "p252_tree_level_timings": (c_int, [c_void_p, c_void_p, c_int, ctypes.POINTER(c_int), ctypes.POINTER(ctypes.c_float)]),
     "p252_dist_unique_id": (c_int, [c_void_p]),
     "p252_dist_init": (c_int, [c_void_p, c_void_p, c_int, c_int]),

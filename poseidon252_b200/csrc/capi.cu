@@ -78,6 +78,9 @@ struct p252_ctx {
     std::vector<char> level_gathered;
     int timed_levels = 0;
     cudaEvent_t ev_tree_end = nullptr;
+    // device scratch of p252_merkle_update_batch (plan of DEVICE calls, staged groups of HOST calls); grows on demand
+    void* upd_scratch = nullptr;
+    size_t upd_scratch_bytes = 0;
 };
 
 #define P252_LOCK(ctx) std::lock_guard<std::recursive_mutex> lock__((ctx)->mu)
@@ -402,6 +405,7 @@ void p252_destroy(p252_ctx* ctx) {
         for (cudaEvent_t ev : {le.k0, le.k1, le.g0, le.g1})
             if (ev) cudaEventDestroy(ev);
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);   // pending host functions reference h_counter
+    if (ctx->upd_scratch) cudaFree(ctx->upd_scratch);
     if (ctx->d_counter) cudaFree(ctx->d_counter);
     if (ctx->h_counter) cudaFreeHost(ctx->h_counter);
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -878,6 +882,175 @@ int p252_merkle_verify_batch(p252_ctx* ctx, int arity, int depth, const p252_fr*
         *n_failed = bad;
     }
     return rc;
+}
+
+// ---- incremental Merkle updates ---------------------------------------------------------------------------------
+// The context's update scratch grows on demand and is never shrunk, so a repeat call with the same or a smaller batch
+// allocates nothing (and a P252_ASYNC call stays asynchronous).
+static int update_scratch(p252_ctx* ctx, size_t bytes, void** out) {
+    if (ctx->upd_scratch_bytes < bytes) {
+        if (ctx->upd_scratch) {
+            CU(cudaStreamSynchronize(ctx->stream));      // earlier calls may still use it
+            CU(cudaFree(ctx->upd_scratch));
+            ctx->upd_scratch = nullptr;
+            ctx->upd_scratch_bytes = 0;
+        }
+        CU(cudaMalloc(&ctx->upd_scratch, bytes));
+        ctx->upd_scratch_bytes = bytes;
+    }
+    *out = ctx->upd_scratch;
+    return P252_OK;
+}
+
+// DEVICE: everything is enqueued on the context stream -- planning (p252::launch_merkle_update_plan) and then one
+// hash launch per level, sized by min(k, level size); each kernel reads its level's real list length on the device.
+static int merkle_update_device(p252_ctx* ctx, int arity, int depth, const p252_fr* tag, p252_fr* leaves, size_t n_leaves,
+                                p252_fr* nodes, const uint64_t* leaf_idx, const p252_fr* values, size_t k,
+                                size_t* n_rejected) {
+    const int s = arity == 4 ? 2 : 1;
+    p252::MerkleUpdatePlan plan = p252::merkle_update_layout(nullptr, k, s, (uint32_t)depth, n_leaves);
+    void* scratch = nullptr;
+    int rc = update_scratch(ctx, plan.total_bytes, &scratch);
+    if (rc != P252_OK) return rc;
+    plan = p252::merkle_update_layout(scratch, k, s, (uint32_t)depth, n_leaves);
+    if (n_rejected && (rc = counter_begin(ctx)) != P252_OK) return rc;
+    cudaError_t le = p252::launch_merkle_update_plan(plan, leaf_idx, values, k, s, (uint32_t)depth, n_leaves, leaves,
+                                                     n_rejected ? ctx->d_counter : nullptr, ctx->stream);
+    if (le != cudaSuccess) return fail_cuda(ctx, le, "merkle update plan");
+    ctx->launches += 2;
+    const p252_fr* below = leaves;
+    p252_fr* level = nodes;
+    for (int l = 0; l < depth; ++l) {
+        const size_t m = n_leaves >> (s * (l + 1));   // nodes of level l + 1
+        le = p252::launch_merkle_update(limbs(tag), arity, below, plan.lists[l], plan.lists[l], level, std::min(k, m),
+                                        plan.counts + l, m, ctx->coop_max, ctx->stream);
+        if (le != cudaSuccess) return fail_cuda(ctx, le, "kernel launch");
+        ctx->launches++;
+        below = level;
+        level += m;
+    }
+    return counter_end(ctx, n_rejected);
+}
+
+// HOST: only the dirty paths travel.  The children groups of every dirty parent are staged with one H2D (level 1:
+// leaves with the new values applied; above: the current nodes, whose dirty entries the level below overwrites on the
+// device), every level's kernel writes its parents into their slots among the next level's staged groups (the top
+// level into a one-slot buffer), one D2H brings the groups back, and only then are the caller's arrays written.
+static int merkle_update_host(p252_ctx* ctx, int arity, int depth, const p252_fr* tag, p252_fr* leaves, size_t n_leaves,
+                              p252_fr* nodes, const uint64_t* leaf_idx, const p252_fr* values, size_t k) {
+    const int s = arity == 4 ? 2 : 1;
+    const size_t A = (size_t)arity;
+    // dedupe: stable order by index, the last occurrence of an index wins
+    std::vector<uint32_t> ord(k);
+    for (size_t i = 0; i < k; ++i) ord[i] = (uint32_t)i;
+    std::stable_sort(ord.begin(), ord.end(), [&](uint32_t a, uint32_t b) { return leaf_idx[a] < leaf_idx[b]; });
+    std::vector<uint32_t> upd;   // batch positions of the surviving writes, by increasing leaf index
+    for (size_t j = 0; j < k; ++j)
+        if (j + 1 == k || leaf_idx[ord[j + 1]] != leaf_idx[ord[j]]) upd.push_back(ord[j]);
+    // dirty parents per level: list[l] = unique(list[l-1] >> log2(arity)), list[0] = the updated leaves
+    std::vector<std::vector<uint64_t>> list((size_t)depth + 1);
+    for (uint32_t u : upd) list[0].push_back(leaf_idx[u]);
+    for (int l = 1; l <= depth; ++l)
+        for (uint64_t c : list[(size_t)l - 1])
+            if (list[(size_t)l].empty() || list[(size_t)l].back() != (c >> s)) list[(size_t)l].push_back(c >> s);
+    // staging layout (scalars): region[l] = |list[l]| groups of `arity` children for l = 1..depth, then the root slot;
+    // then the write-slot indices of every level (u64)
+    std::vector<size_t> region((size_t)depth + 2, 0), widx_off((size_t)depth + 2, 0);
+    for (int l = 1; l <= depth; ++l) {
+        region[(size_t)l + 1] = region[(size_t)l] + list[(size_t)l].size() * A;
+        widx_off[(size_t)l + 1] = widx_off[(size_t)l] + list[(size_t)l].size();
+    }
+    const size_t n_stage = region[(size_t)depth + 1] + 1, n_widx = widx_off[(size_t)depth + 1];
+    const size_t stage_bytes = n_stage * sizeof(p252_fr);
+    std::vector<p252_fr> stage(n_stage);
+    std::vector<uint64_t> widx(n_widx);
+    std::vector<size_t> off((size_t)depth + 1, 0);   // offset of internal level l inside nodes
+    for (int l = 2; l <= depth; ++l) off[(size_t)l] = off[(size_t)l - 1] + (n_leaves >> (s * (l - 1)));
+    for (int l = 1; l <= depth; ++l) {
+        const std::vector<uint64_t>& L = list[(size_t)l];
+        const p252_fr* src = (l == 1) ? leaves : nodes + off[(size_t)l - 1];
+        for (size_t j = 0; j < L.size(); ++j) memcpy(&stage[region[(size_t)l] + j * A], src + L[j] * A, A * sizeof(p252_fr));
+        if (l == depth) {
+            widx[widx_off[(size_t)l]] = 0;
+            continue;
+        }
+        const std::vector<uint64_t>& up = list[(size_t)l + 1];
+        for (size_t j = 0, r = 0; j < L.size(); ++j) {
+            while (up[r] != (L[j] >> s)) ++r;
+            widx[widx_off[(size_t)l] + j] = r * A + (L[j] & (A - 1));
+        }
+    }
+    for (size_t j = 0, r = 0; j < upd.size(); ++j) {   // the new leaf values
+        const uint64_t i = leaf_idx[upd[j]];
+        while (list[1][r] != (i >> s)) ++r;
+        stage[region[1] + r * A + (i & (A - 1))] = values[upd[j]];
+    }
+    std::vector<uint8_t> h(stage_bytes + n_widx * 8);
+    memcpy(h.data(), stage.data(), stage_bytes);
+    memcpy(h.data() + stage_bytes, widx.data(), n_widx * 8);
+    void* scratch = nullptr;
+    int rc = update_scratch(ctx, h.size(), &scratch);
+    if (rc != P252_OK) return rc;
+    p252_fr* d_stage = static_cast<p252_fr*>(scratch);
+    const uint64_t* d_widx = reinterpret_cast<const uint64_t*>(static_cast<uint8_t*>(scratch) + stage_bytes);
+    auto body = [&]() -> int {
+        CU(cudaMemcpyAsync(scratch, h.data(), h.size(), cudaMemcpyHostToDevice, ctx->stream));
+        for (int l = 1; l <= depth; ++l) {
+            const size_t n = list[(size_t)l].size();
+            p252_fr* out = d_stage + region[(size_t)l + 1];   // the next level's groups, or the root slot
+            cudaError_t le = p252::launch_merkle_update(limbs(tag), arity, d_stage + region[(size_t)l], nullptr,
+                                                        d_widx + widx_off[(size_t)l], out, n, nullptr, n, ctx->coop_max,
+                                                        ctx->stream);
+            if (le != cudaSuccess) return fail_cuda(ctx, le, "kernel launch");
+            ctx->launches++;
+        }
+        CU(cudaMemcpyAsync(stage.data() + region[2], d_stage + region[2], (n_stage - region[2]) * sizeof(p252_fr),
+                           cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaStreamSynchronize(ctx->stream));
+        return P252_OK;
+    };
+    rc = body();
+    if (rc != P252_OK) {
+        cudaStreamSynchronize(ctx->stream);   // nothing may still read or write the staging vectors
+        cudaGetLastError();
+        return rc;
+    }
+    // all device work succeeded: write the caller's tree
+    for (int l = 1; l < depth; ++l) {
+        const std::vector<uint64_t>& L = list[(size_t)l];
+        for (size_t j = 0; j < L.size(); ++j)
+            nodes[off[(size_t)l] + L[j]] = stage[region[(size_t)l + 1] + widx[widx_off[(size_t)l] + j]];
+    }
+    nodes[off[(size_t)depth]] = stage[region[(size_t)depth + 1]];
+    for (uint32_t u : upd) leaves[leaf_idx[u]] = values[u];
+    return P252_OK;
+}
+
+int p252_merkle_update_batch(p252_ctx* ctx, int arity, p252_fr* leaves, size_t n_leaves, p252_fr* nodes,
+                             const uint64_t* leaf_idx, const p252_fr* values, size_t k, size_t* n_rejected, int flags) {
+    if (!ctx || !leaves || !nodes || ((!leaf_idx || !values) && k)) return P252_ERR_INVALID_ARGUMENT;
+    int depth = 0;
+    int rc = tree_depth(arity, n_leaves, &depth);
+    if (rc != P252_OK) return rc;
+    if (k > 0xffffffffull) return P252_ERR_INVALID_ARGUMENT;   // batch positions are 32-bit
+    p252_fr tag;
+    if ((rc = p252_hash_tag(merkle_domain(arity), (size_t)arity, 1, &tag)) != P252_OK) return rc;
+    P252_LOCK(ctx);
+    DeviceGuard g(ctx->device);
+    if (n_rejected) *n_rejected = 0;
+    if (flags & P252_MEM_DEVICE) {
+        if (!aligned16(leaves) || !aligned16(nodes) || !aligned16(values) || (reinterpret_cast<uintptr_t>(leaf_idx) & 7))
+            return P252_ERR_INVALID_ARGUMENT;
+        if (k == 0) return P252_OK;
+        rc = merkle_update_device(ctx, arity, depth, &tag, leaves, n_leaves, nodes, leaf_idx, values, k, n_rejected);
+        if (rc != P252_OK) return rc;
+        if (!(flags & P252_ASYNC)) CU(cudaStreamSynchronize(ctx->stream));
+        return P252_OK;
+    }
+    for (size_t i = 0; i < k; ++i)
+        if (leaf_idx[i] >= n_leaves) return P252_ERR_INVALID_ARGUMENT;   // before anything is written
+    if (k == 0) return P252_OK;
+    return merkle_update_host(ctx, arity, depth, &tag, leaves, n_leaves, nodes, leaf_idx, values, k);
 }
 
 // ---- multi-GPU ------------------------------------------------------------------------------------------

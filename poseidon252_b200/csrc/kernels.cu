@@ -13,6 +13,10 @@
 
 #include <cstdlib>
 
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_select.cuh>
+#include <thrust/iterator/transform_iterator.h>
+
 #include "hades_device.cuh"
 
 namespace p252 {
@@ -474,6 +478,195 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) k_merkle_verify(FrArg ta
     }
 }
 
+// ---- incremental Merkle updates: one launch per dirty level -------------------------------------------------------
+// Entry j (< n = min(*d_count, bound), or bound when d_count is null) of a level's work list reads the `arity` children
+// of group g = read_idx[j] (read_idx null: g = j) at below + g*arity*32, digests them on the Merkle tag and stores the
+// parent at out + write_idx[j]*32.  Entries with g >= n_groups are skipped: the device plan ends every list with one
+// out-of-range sentinel.  The device path passes the dirty parent list as both indices (read the children of p, write
+// p); the host path reads staged groups in list order and writes each parent into its slot among the next level's
+// staged groups.
+__device__ __forceinline__ size_t update_count(size_t bound, const int64_t* d_count) {
+    if (!d_count) return bound;
+    const int64_t c = *d_count;
+    return c < 0 ? 0 : ((size_t)c < bound ? (size_t)c : bound);
+}
+
+// one state per thread; the children of a group are `arity` consecutive scalars (arity 4: one aligned 128-byte line)
+template <int kLog2Arity>
+__global__ void __launch_bounds__(kThreads, kMinBlocks) k_merkle_update(FrArg tag, const uint8_t* __restrict__ below,
+                                                                        const uint64_t* __restrict__ read_idx,
+                                                                        const uint64_t* __restrict__ write_idx,
+                                                                        uint8_t* __restrict__ out, size_t bound,
+                                                                        const int64_t* __restrict__ d_count, uint64_t n_groups) {
+    constexpr int kArity = 1 << kLog2Arity;
+    P252_STAGE_TABLES
+    const size_t j = (size_t)blockIdx.x * kThreads + threadIdx.x;
+    if (j >= update_count(bound, d_count)) return;
+    const uint64_t g = read_idx ? read_idx[j] : (uint64_t)j;
+    if (g >= n_groups) return;
+    const uint8_t* src = below + g * (kArity * 32);
+    uint32_t s[5][8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) s[0][k] = tag.l[k];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+        if (q < kArity) {
+            load_fr(s[1 + q], src + q * 32);
+        } else {
+#pragma unroll
+            for (int k = 0; k < 8; ++k) s[1 + q][k] = 0;
+        }
+    }
+    hades_permute(s, 0x2u P252_TAB_PASS);              // a Merkle digest reads lane 1 only
+    store_fr(out + write_idx[j] * 32, s[1]);
+}
+
+// the same with five threads per state (hades_permute_coop): 6 entries per warp, thread li loads lane li of the state
+template <int kLog2Arity>
+__global__ void __launch_bounds__(kThreads) k_merkle_update_coop(FrArg tag, const uint8_t* __restrict__ below,
+                                                                 const uint64_t* __restrict__ read_idx,
+                                                                 const uint64_t* __restrict__ write_idx,
+                                                                 uint8_t* __restrict__ out, size_t bound,
+                                                                 const int64_t* __restrict__ d_count, uint64_t n_groups) {
+    constexpr int kArity = 1 << kLog2Arity;
+    const int lane = threadIdx.x & 31;
+    const int grp = lane / 5, li = lane - grp * 5, g0 = grp * 5;
+    const size_t warp_global = (size_t)blockIdx.x * kWarps + (threadIdx.x >> 5);
+    const size_t j = warp_global * kCoopItemsPerWarp + grp;
+    const size_t n = update_count(bound, d_count);
+    if (warp_global * kCoopItemsPerWarp >= n) return;            // whole warp idle (n is warp-uniform)
+    const uint64_t g = (grp < kCoopItemsPerWarp && j < n) ? (read_idx ? read_idx[j] : (uint64_t)j) : n_groups;
+    const bool live = g < n_groups;                              // idle threads still take part in the shuffles
+    double crow[5];
+#pragma unroll
+    for (int q = 0; q < 5; ++q) crow[q] = (double)(HADES_LAMBDA / (uint32_t)(li + q + 5));
+    uint32_t s[8];
+    if (li == 0) {
+#pragma unroll
+        for (int k = 0; k < 8; ++k) s[k] = tag.l[k];
+    } else if (live && li <= kArity) {
+        load_fr(s, below + g * (kArity * 32) + (size_t)(li - 1) * 32);
+    } else {
+#pragma unroll
+        for (int k = 0; k < 8; ++k) s[k] = 0;
+    }
+    hades_permute_coop(s, li, g0, crow);
+    if (live && li == 1) store_fr(out + write_idx[j] * 32, s);
+}
+
+// ---- device-side planning of an update batch ------------------------------------------------------------------------
+// keys[j] = leaf_idx[j], or n_leaves when it is outside the tree (counted into *n_rejected); pos[j] = j.
+__global__ void __launch_bounds__(256) k_update_keys(const uint64_t* __restrict__ leaf_idx, size_t k, uint64_t n_leaves,
+                                                     uint64_t* __restrict__ keys, uint32_t* __restrict__ pos,
+                                                     unsigned long long* __restrict__ n_rejected) {
+    const size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const bool in = j < k;
+    bool bad = false;
+    if (in) {
+        const uint64_t i = leaf_idx[j];
+        bad = i >= n_leaves;
+        keys[j] = bad ? n_leaves : i;
+        pos[j] = (uint32_t)j;
+    }
+    if (n_rejected) {                                            // one atomic per warp that saw a rejected index
+        const unsigned b = __ballot_sync(0xffffffffu, bad);
+        if (b && (threadIdx.x & 31) == 0) atomicAdd(n_rejected, (unsigned long long)__popc(b));
+    }
+}
+
+// After the stable sort the last entry of every run of equal keys is the batch's last write to that leaf.
+__global__ void __launch_bounds__(256) k_update_leaves(const uint64_t* __restrict__ keys, const uint32_t* __restrict__ pos,
+                                                       size_t k, uint64_t n_leaves, const uint8_t* __restrict__ values,
+                                                       uint8_t* __restrict__ leaves) {
+    const size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= k) return;
+    const uint64_t key = keys[j];
+    if (key >= n_leaves || (j + 1 < k && keys[j + 1] == key)) return;
+    uint32_t v[8];
+    load_fr(v, values + (size_t)pos[j] * 32);
+    store_fr(leaves + key * 32, v);
+}
+
+// parent of a sorted list entry; everything at or beyond `limit` (rejected leaves, the sentinel) maps to the sentinel
+struct ParentOf {
+    uint64_t limit;
+    int shift;
+    __host__ __device__ uint64_t operator()(uint64_t x) const { return x >= limit ? kUpdateSentinel : x >> shift; }
+};
+
+MerkleUpdatePlan merkle_update_layout(void* scratch, size_t k, int log2_arity, uint32_t depth, uint64_t n_leaves) {
+    MerkleUpdatePlan p{};
+    size_t off = 0;
+    auto take = [&](size_t bytes) {
+        void* q = scratch ? static_cast<uint8_t*>(scratch) + off : nullptr;
+        off += (bytes + 255) / 256 * 256;
+        return q;
+    };
+    p.keys_in = static_cast<uint64_t*>(take(k * 8));
+    p.keys_out = static_cast<uint64_t*>(take(k * 8));
+    p.pos_in = static_cast<uint32_t*>(take(k * 4));
+    p.pos_out = static_cast<uint32_t*>(take(k * 4));
+    p.counts = static_cast<int64_t*>(take((size_t)depth * 8));
+    // list l (parents at level l + 1) holds at most min(entries of the list below, level size + 1 sentinel) entries
+    size_t lists_bytes = 0, cap = k;
+    uint64_t m = n_leaves;
+    for (uint32_t l = 0; l < depth; ++l) {
+        m >>= log2_arity;
+        cap = cap < m + 1 ? cap : (size_t)(m + 1);
+        p.list_cap[l] = cap;
+        lists_bytes += cap * 8;
+    }
+    p.lists_bytes = lists_bytes;
+    uint64_t* lists = static_cast<uint64_t*>(take(lists_bytes));
+    for (uint32_t l = 0; l < depth; ++l) {
+        p.lists[l] = lists;
+        if (lists) lists += p.list_cap[l];
+    }
+    // CUB temporary storage: the larger of the sort's and the widest unique's (sizes only, no device work)
+    int end_bit = 1;
+    while (end_bit < 64 && (n_leaves >> end_bit) != 0) ++end_bit;   // keys <= n_leaves
+    p.end_bit = end_bit;
+    size_t sort_bytes = 0, uniq_bytes = 0;
+    cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, p.keys_in, p.keys_out, p.pos_in, p.pos_out, k, 0, end_bit);
+    auto it = thrust::make_transform_iterator(p.keys_out, ParentOf{n_leaves, log2_arity});
+    cub::DeviceSelect::Unique(nullptr, uniq_bytes, it, p.lists[0], p.counts, (int64_t)k);
+    p.temp_bytes = sort_bytes > uniq_bytes ? sort_bytes : uniq_bytes;
+    p.temp = take(p.temp_bytes);
+    p.total_bytes = off;
+    return p;
+}
+
+cudaError_t launch_merkle_update_plan(const MerkleUpdatePlan& p, const uint64_t* leaf_idx, const void* values, size_t k,
+                                      int log2_arity, uint32_t depth, uint64_t n_leaves, void* leaves,
+                                      unsigned long long* n_rejected, cudaStream_t st) {
+    const unsigned grid = (unsigned)((k + 255) / 256);
+    k_update_keys<<<grid, 256, 0, st>>>(leaf_idx, k, n_leaves, p.keys_in, p.pos_in, n_rejected);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    size_t tb = p.temp_bytes;
+    e = cub::DeviceRadixSort::SortPairs(p.temp, tb, p.keys_in, p.keys_out, p.pos_in, p.pos_out, k, 0, p.end_bit, st);
+    if (e != cudaSuccess) return e;
+    k_update_leaves<<<grid, 256, 0, st>>>(p.keys_out, p.pos_out, k, n_leaves, static_cast<const uint8_t*>(values),
+                                          static_cast<uint8_t*>(leaves));
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    // Entries past a list's unique count stay at the sentinel, so the next level's unique may read the whole
+    // capacity: the sentinels collapse into one trailing entry.
+    if ((e = cudaMemsetAsync(p.lists[0], 0xff, p.lists_bytes, st)) != cudaSuccess) return e;
+    uint64_t m = n_leaves;
+    for (uint32_t l = 0; l < depth; ++l) {
+        tb = p.temp_bytes;
+        if (l == 0)
+            e = cub::DeviceSelect::Unique(p.temp, tb, thrust::make_transform_iterator(p.keys_out, ParentOf{n_leaves, log2_arity}),
+                                          p.lists[0], p.counts, (int64_t)k, st);
+        else
+            e = cub::DeviceSelect::Unique(p.temp, tb, thrust::make_transform_iterator(p.lists[l - 1], ParentOf{m, log2_arity}),
+                                          p.lists[l], p.counts + l, (int64_t)p.list_cap[l - 1], st);
+        if (e != cudaSuccess) return e;
+        m >>= log2_arity;
+    }
+    return cudaSuccess;
+}
+
 // ---- host-callable launchers -------------------------------------------------------------------
 static inline FrArg to_arg(const uint64_t tag[4]) {
     FrArg a;
@@ -617,6 +810,27 @@ cudaError_t launch_merkle_verify(const uint64_t tag[4], const uint64_t root[4], 
     else
         k_merkle_verify<1><<<grid_for(n), kThreads, 0, st>>>(to_arg(tag), to_arg(root), static_cast<const uint8_t*>(leaf_items),
                                                              leaf_idx, static_cast<const uint8_t*>(paths), n, depth, ok, n_failed);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_merkle_update(const uint64_t tag[4], int arity, const void* below, const uint64_t* read_idx,
+                                 const uint64_t* write_idx, void* out, size_t bound, const int64_t* d_count,
+                                 uint64_t n_groups, size_t coop_max, cudaStream_t st) {
+    if (bound == 0) return cudaSuccess;
+    const uint8_t* b = static_cast<const uint8_t*>(below);
+    uint8_t* o = static_cast<uint8_t*>(out);
+    if (bound <= coop_max) {                     // the same choice as launch_digest
+        const size_t warps = (bound + kCoopItemsPerWarp - 1) / kCoopItemsPerWarp;
+        const unsigned grid = (unsigned)((warps + kWarps - 1) / kWarps);
+        if (arity == 4)
+            k_merkle_update_coop<2><<<grid, kThreads, 0, st>>>(to_arg(tag), b, read_idx, write_idx, o, bound, d_count, n_groups);
+        else
+            k_merkle_update_coop<1><<<grid, kThreads, 0, st>>>(to_arg(tag), b, read_idx, write_idx, o, bound, d_count, n_groups);
+    } else if (arity == 4) {
+        k_merkle_update<2><<<grid_for(bound), kThreads, 0, st>>>(to_arg(tag), b, read_idx, write_idx, o, bound, d_count, n_groups);
+    } else {
+        k_merkle_update<1><<<grid_for(bound), kThreads, 0, st>>>(to_arg(tag), b, read_idx, write_idx, o, bound, d_count, n_groups);
+    }
     return cudaGetLastError();
 }
 

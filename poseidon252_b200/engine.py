@@ -368,6 +368,56 @@ class Engine:
     def last_verify_failures(self):
         return int(getattr(self, "_vfail", ctypes.c_size_t(0)).value)
 
+    # -- incremental Merkle updates ---------------------------------------------------------------
+    def _inplace(self, name, x, rows):
+        """A buffer the call writes in place: it must already be exactly what native code writes through (a copy would
+        silently lose the update)."""
+        if _is_torch(x):
+            if not x.is_cuda or x.device.index != self.device:
+                raise EngineError(-1, "%s is not on cuda:%d" % (name, self.device))
+            ok = str(x.dtype) in ("torch.int64", "torch.uint64") and x.is_contiguous()
+        else:
+            ok = isinstance(x, np.ndarray) and x.dtype in (np.uint64, np.int64) and x.flags.c_contiguous and \
+                x.flags.writeable
+        if not ok:
+            raise EngineError(-1, "%s must be a writable C-contiguous uint64/int64 array or tensor (updated in place)" % name)
+        if tuple(x.shape) != (rows, 4):
+            raise EngineError(-1, "%s must have shape (%d, 4), got %s" % (name, rows, tuple(x.shape)))
+        return self._ptr(x), (_native.MEM_DEVICE if _is_torch(x) else _native.MEM_HOST)
+
+    def merkle_update_batch(self, leaves, nodes, leaf_idx, values, arity=4, async_=False):
+        """Write values[j] to leaf leaf_idx[j] (the last occurrence of a repeated index wins) and rehash only the
+        dirty paths, in place: afterwards leaves / nodes equal merkle_build of the updated leaves.  Returns
+        (leaves, nodes).  Host arrays: an index outside the tree raises before anything is written.  Device tensors:
+        such entries are skipped and counted (last_update_rejected(); after an async_ call, sync() first)."""
+        n_leaves = int(leaves.shape[0]) if getattr(leaves, "ndim", 0) == 2 else -1
+        ni = ctypes.c_size_t(0)
+        if n_leaves < 0:
+            raise EngineError(-1, "leaves must have shape (n_leaves, 4)")
+        self._check(self._lib.p252_merkle_tree_nodes(int(arity), n_leaves, ctypes.byref(ni), None))
+        lp, flags = self._inplace("leaves", leaves, n_leaves)
+        np_, f2 = self._inplace("nodes", nodes, int(ni.value))
+        if getattr(values, "ndim", 0) != 2:
+            raise EngineError(-1, "values must have shape (k, 4)")
+        vp, vlead, f3, vk = self._in(values, (4,))
+        if not (flags == f2 == f3) or _is_torch(leaf_idx) != _is_torch(leaves):
+            raise EngineError(-1, "all buffers must live in the same memory space")
+        ip, k, ik = self._idx(leaf_idx, leaves)
+        if k != vlead[0]:
+            raise EngineError(-1, "leaf_idx has %d entries but values has %d rows" % (k, vlead[0]))
+        if flags == _native.MEM_DEVICE:
+            self._fence_torch()
+        # written after the stream reaches it for device calls: keep it alive on the engine
+        self._ufail = ctypes.c_size_t(0)
+        self._check(self._lib.p252_merkle_update_batch(self._ctx, int(arity), lp, n_leaves, np_, ip, vp, k,
+                                                       ctypes.byref(self._ufail),
+                                                       flags | (_native.ASYNC if async_ and flags else 0)))
+        return leaves, nodes
+
+    def last_update_rejected(self):
+        """Entries of the last merkle_update_batch on device tensors whose leaf index was outside the tree."""
+        return int(getattr(self, "_ufail", ctypes.c_size_t(0)).value)
+
     def set_small_batch_max(self, max_items):
         """Digest batches up to `max_items` items use the lane-split (5 threads per state) kernel; 0 disables it."""
         self._check(self._lib.p252_set_small_batch_max(self._ctx, int(max_items)))

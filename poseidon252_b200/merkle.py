@@ -34,6 +34,13 @@ def verify_batch(leaf_items, leaf_idx, paths, root, arity=4, engine=None, async_
     return eng.merkle_verify_batch(leaf_items, leaf_idx, paths, root, arity=arity, async_=async_)
 
 
+def update_batch(leaves, nodes, leaf_idx, values, arity=4, engine=None, async_=False):
+    """Overwrite the leaves `leaf_idx` with `values` (last occurrence wins) and rehash only their paths, in place:
+    afterwards (leaves, nodes) equal a rebuild.  Returns (leaves, nodes)."""
+    eng = engine or default_engine(leaves.device.index if hasattr(leaves, "is_cuda") else 0)
+    return eng.merkle_update_batch(leaves, nodes, leaf_idx, values, arity=arity, async_=async_)
+
+
 def positions(leaf_idx, depth, arity=4):
     """Offset of the path node inside its sibling group at every level (the `positions` of an Opening)."""
     out, i = [], int(leaf_idx)
