@@ -250,35 +250,45 @@ int run_host_pipeline(p252_ctx* ctx, std::vector<Io>& ios, size_t n, Launch laun
     return P252_OK;
 }
 
-int finish_device_call(p252_ctx* ctx, cudaError_t le, int flags) {
-    if (le != cudaSuccess) return fail_cuda(ctx, le, "kernel launch");
-    ctx->launches++;
-    if (!(flags & P252_ASYNC)) CU(cudaStreamSynchronize(ctx->stream));
+// Counts n enqueued kernels, or turns a failed launch into a status.
+int count_launch(p252_ctx* ctx, cudaError_t le, const char* what = "kernel launch", int n = 1) {
+    if (le != cudaSuccess) return fail_cuda(ctx, le, what);
+    ctx->launches += n;
     return P252_OK;
 }
 
-// DEVICE-buffer calls that count failures on the device: zero the counter before the launch ...
-int counter_begin(p252_ctx* ctx) {
-    CU(cudaMemsetAsync(ctx->d_counter, 0, sizeof(unsigned long long), ctx->stream));
-    return P252_OK;
-}
 void CUDART_CB publish_counter(void* arg) {
     auto* pr = static_cast<std::pair<const unsigned long long*, size_t*>*>(arg);
     *pr->second = (size_t)*pr->first;
     delete pr;
 }
-// ... and after it copy the counter to the pinned mirror and from there to the caller's size_t (a host function on
-// the stream, so that P252_ASYNC callers see it after p252_sync).
-int counter_end(p252_ctx* ctx, size_t* n_failed) {
-    if (!n_failed) return P252_OK;
-    CU(cudaMemcpyAsync(ctx->h_counter, ctx->d_counter, sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
-    auto* pr = new std::pair<const unsigned long long*, size_t*>(ctx->h_counter, n_failed);
-    cudaError_t e = cudaLaunchHostFunc(ctx->stream, publish_counter, pr);
-    if (e != cudaSuccess) {
-        delete pr;
-        return fail_cuda(ctx, e, "cudaLaunchHostFunc");
+
+// Every DEVICE-buffer call: launch(counter) enqueues the work on the context stream, counts its launches
+// (count_launch) and returns a status.  With n_failed, counter is the context's device counter, zeroed before the
+// launch and afterwards copied to the pinned mirror and from there to *n_failed by a host function on the stream, so
+// that P252_ASYNC callers see it after p252_sync; without, counter is null.  Synchronises unless P252_ASYNC.
+template <typename Launch>
+int device_call(p252_ctx* ctx, int flags, size_t* n_failed, Launch launch) {
+    if (n_failed) CU(cudaMemsetAsync(ctx->d_counter, 0, sizeof(unsigned long long), ctx->stream));
+    const int rc = launch(n_failed ? ctx->d_counter : nullptr);
+    if (rc != P252_OK) return rc;
+    if (n_failed) {
+        CU(cudaMemcpyAsync(ctx->h_counter, ctx->d_counter, sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+        auto* pr = new std::pair<const unsigned long long*, size_t*>(ctx->h_counter, n_failed);
+        cudaError_t e = cudaLaunchHostFunc(ctx->stream, publish_counter, pr);
+        if (e != cudaSuccess) {
+            delete pr;
+            return fail_cuda(ctx, e, "cudaLaunchHostFunc");
+        }
     }
+    if (!(flags & P252_ASYNC)) CU(cudaStreamSynchronize(ctx->stream));
     return P252_OK;
+}
+
+// HOST calls that write one ok byte per item: once the call succeeded, *n_failed (optional) = the zero bytes.
+int count_failed(int rc, const uint8_t* ok, size_t n, size_t* n_failed) {
+    if (rc == P252_OK && n_failed) *n_failed = (size_t)std::count(ok, ok + n, 0);
+    return rc;
 }
 
 uint64_t domain_sep(int domain, bool* ok) {
@@ -294,6 +304,49 @@ uint64_t domain_sep(int domain, bool* ok) {
 }
 
 const uint64_t* limbs(const p252_fr* f) { return f->l; }
+
+// Tag of one Merkle node: Hash::digest(Domain::Merkle2 | Merkle4, `arity` children), src/hash.rs:22-31.
+int merkle_tag(int arity, p252_fr* tag) {
+    if (arity != 2 && arity != 4) return P252_ERR_INVALID_ARGUMENT;
+    return p252_hash_tag(arity == 4 ? P252_DOMAIN_MERKLE4 : P252_DOMAIN_MERKLE2, (size_t)arity, 1, tag);
+}
+
+// A full Merkle tree in the layout p252_merkle_build writes: height 0 is the n_leaves = arity^depth leaves (the
+// caller's `leaves`), heights 1..depth are the internal levels, bottom-up and concatenated in `nodes`; the root
+// (height depth) is the last node.
+struct Tree {
+    int arity, log2_arity, depth;
+    size_t n_leaves, n_internal;
+    p252_fr tag;
+    size_t off[p252::kMaxDepth + 1];   // offset(h), precomputed: the HOST gathers look it up per item and level
+    size_t size(int h) const { return n_leaves >> (log2_arity * h); }
+    // first node of height h inside its buffer: 0 for the leaves, n_internal - 1 for the root
+    size_t offset(int h) const { return off[h]; }
+    template <typename T>
+    T* level(T* leaves, T* nodes, int h) const { return (h == 0 ? leaves : nodes) + offset(h); }
+    // the `arity` children of group g at height h
+    template <typename T>
+    T* group(T* leaves, T* nodes, int h, uint64_t g) const { return level(leaves, nodes, h) + g * (uint64_t)arity; }
+};
+static_assert(p252::kMaxDepth >= 63, "a tree with at most 2^64 - 1 leaves has at most 63 levels");
+
+// P252_ERR_INVALID_ARGUMENT for an arity other than 2 or 4 or fewer than 2 leaves, P252_ERR_IO_PATTERN_VIOLATION when a
+// level is not a multiple of the arity.
+int make_tree(int arity, size_t n_leaves, Tree* t) {
+    int rc = merkle_tag(arity, &t->tag);
+    if (rc != P252_OK) return rc;
+    if (n_leaves < 2) return P252_ERR_INVALID_ARGUMENT;
+    t->arity = arity;
+    t->log2_arity = arity == 4 ? 2 : 1;
+    t->depth = 0;
+    for (size_t m = n_leaves; m > 1; m /= (size_t)arity, ++t->depth)
+        if (m % (size_t)arity) return P252_ERR_IO_PATTERN_VIOLATION;
+    t->n_leaves = n_leaves;
+    t->n_internal = (n_leaves - 1) / (size_t)(arity - 1);
+    t->off[0] = t->off[1] = 0;
+    for (int h = 2; h <= t->depth; ++h) t->off[h] = t->off[h - 1] + t->size(h - 1);
+    return P252_OK;
+}
 
 }  // namespace
 
@@ -562,7 +615,9 @@ static int permute_impl(p252_ctx* ctx, p252_fr* states, size_t n, int flags, boo
     if (flags & P252_MEM_DEVICE) {
         if (!aligned16(states)) return P252_ERR_INVALID_ARGUMENT;
         if (n == 0) return P252_OK;
-        return finish_device_call(ctx, p252::launch_permute(states, n, dense, ctx->coop_max, ctx->stream), flags);
+        return device_call(ctx, flags, nullptr, [&](auto) {
+            return count_launch(ctx, p252::launch_permute(states, n, dense, ctx->coop_max, ctx->stream));
+        });
     }
     std::vector<Io> ios = {{states, states, 160}};
     return run_host_pipeline(ctx, ios, n, [&](void** d, size_t cnt, cudaStream_t st) {
@@ -588,7 +643,9 @@ static int digest_impl(p252_ctx* ctx, const p252_fr* tag, const p252_fr* in, siz
     if (flags & P252_MEM_DEVICE) {
         if (!aligned16(in) || !aligned16(out)) return P252_ERR_INVALID_ARGUMENT;
         if (n == 0) return P252_OK;
-        return finish_device_call(ctx, p252::launch_digest(limbs(tag), in, n, il, out, ol, truncate, ctx->coop_max, ctx->stream), flags);
+        return device_call(ctx, flags, nullptr, [&](auto) {
+            return count_launch(ctx, p252::launch_digest(limbs(tag), in, n, il, out, ol, truncate, ctx->coop_max, ctx->stream));
+        });
     }
     std::vector<Io> ios = {{in, nullptr, in_len * 32}, {nullptr, out, out_len * 32}};
     return run_host_pipeline(ctx, ios, n, [&](void** d, size_t cnt, cudaStream_t st) {
@@ -624,7 +681,9 @@ static int convert_impl(p252_ctx* ctx, const void* in, size_t n, void* out, uint
     if (flags & P252_MEM_DEVICE) {
         if (!aligned16(in) || !aligned16(out)) return P252_ERR_INVALID_ARGUMENT;
         if (n == 0) return P252_OK;
-        return finish_device_call(ctx, p252::launch_convert(in, n, out, ok, from_bytes, ctx->stream), flags);
+        return device_call(ctx, flags, nullptr, [&](auto) {
+            return count_launch(ctx, p252::launch_convert(in, n, out, ok, from_bytes, ctx->stream));
+        });
     }
     std::vector<Io> ios = {{in, nullptr, 32}, {nullptr, out, 32}};
     if (from_bytes && ok) ios.push_back({nullptr, ok, 1});
@@ -654,8 +713,9 @@ int p252_encrypt_batch(p252_ctx* ctx, const p252_fr* msg, size_t n, size_t L, co
         if (!aligned16(msg) || !aligned16(secret_uv) || !aligned16(nonce) || !aligned16(cipher))
             return P252_ERR_INVALID_ARGUMENT;
         if (n == 0) return P252_OK;
-        return finish_device_call(
-            ctx, p252::launch_encrypt(limbs(&tag), msg, n, l32, secret_uv, nonce, cipher, ctx->stream), flags);
+        return device_call(ctx, flags, nullptr, [&](auto) {
+            return count_launch(ctx, p252::launch_encrypt(limbs(&tag), msg, n, l32, secret_uv, nonce, cipher, ctx->stream));
+        });
     }
     std::vector<Io> ios = {{msg, nullptr, L * 32}, {secret_uv, nullptr, 64}, {nonce, nullptr, 32},
                            {nullptr, cipher, (L + 1) * 32}};
@@ -678,26 +738,17 @@ int p252_decrypt_batch(p252_ctx* ctx, const p252_fr* cipher, size_t n, size_t L,
             return P252_ERR_INVALID_ARGUMENT;
         if (n_failed) *n_failed = 0;
         if (n == 0) return P252_OK;
-        if (n_failed && (rc = counter_begin(ctx)) != P252_OK) return rc;
-        cudaError_t le = p252::launch_decrypt(limbs(&tag), cipher, n, l32, secret_uv, nonce, msg, ok,
-                                              n_failed ? ctx->d_counter : nullptr, ctx->stream);
-        if (le != cudaSuccess) return fail_cuda(ctx, le, "kernel launch");
-        ctx->launches++;
-        if ((rc = counter_end(ctx, n_failed)) != P252_OK) return rc;
-        if (!(flags & P252_ASYNC)) CU(cudaStreamSynchronize(ctx->stream));
-        return P252_OK;
+        return device_call(ctx, flags, n_failed, [&](unsigned long long* failed) {
+            return count_launch(ctx, p252::launch_decrypt(limbs(&tag), cipher, n, l32, secret_uv, nonce, msg, ok, failed,
+                                                          ctx->stream));
+        });
     }
     std::vector<Io> ios = {{cipher, nullptr, (L + 1) * 32}, {secret_uv, nullptr, 64}, {nonce, nullptr, 32},
                            {nullptr, msg, L * 32}, {nullptr, ok, 1}};
     rc = run_host_pipeline(ctx, ios, n, [&](void** d, size_t cnt, cudaStream_t st) {
         return p252::launch_decrypt(limbs(&tag), d[0], cnt, l32, d[1], d[2], d[3], static_cast<uint8_t*>(d[4]), nullptr, st);
     }, /*wipe=*/true);
-    if (rc == P252_OK && n_failed) {
-        size_t bad = 0;
-        for (size_t i = 0; i < n; ++i) bad += ok[i] ? 0 : 1;
-        *n_failed = bad;
-    }
-    return rc;
+    return count_failed(rc, ok, n, n_failed);
 }
 
 // ---- arity-4 Merkle tree ------------------------------------------------------------------------------
@@ -705,25 +756,12 @@ int p252_merkle4_level(p252_ctx* ctx, const p252_fr* children, size_t n_parents,
     return p252_hash_batch(ctx, P252_DOMAIN_MERKLE4, children, n_parents, 4, parents, 1, flags);
 }
 
-static int merkle_domain(int arity) {
-    return arity == 4 ? P252_DOMAIN_MERKLE4 : (arity == 2 ? P252_DOMAIN_MERKLE2 : -1);
-}
-
 int p252_merkle_tree_nodes(int arity, size_t n_leaves, size_t* n_internal, int* n_levels) {
-    if (merkle_domain(arity) < 0) return P252_ERR_INVALID_ARGUMENT;
-    const size_t A = (size_t)arity;
-    size_t m = n_leaves, total = 0;
-    int lv = 0;
-    if (m == 0) return P252_ERR_INVALID_ARGUMENT;
-    while (m > 1) {
-        if (m % A) return P252_ERR_IO_PATTERN_VIOLATION;   // a level that is not a multiple of the arity
-        m /= A;
-        total += m;
-        ++lv;
-    }
-    if (lv == 0) return P252_ERR_INVALID_ARGUMENT;
-    if (n_internal) *n_internal = total;                 // (n_leaves - 1) / (arity - 1)
-    if (n_levels) *n_levels = lv;
+    Tree t;
+    int rc = make_tree(arity, n_leaves, &t);
+    if (rc != P252_OK) return rc;
+    if (n_internal) *n_internal = t.n_internal;
+    if (n_levels) *n_levels = t.depth;
     return P252_OK;
 }
 
@@ -731,59 +769,48 @@ int p252_merkle4_tree_nodes(size_t n_leaves, size_t* n_internal, int* n_levels) 
     return p252_merkle_tree_nodes(4, n_leaves, n_internal, n_levels);
 }
 
-static int merkle_build_device(p252_ctx* ctx, int arity, const p252_fr* leaves, size_t n_leaves, p252_fr* nodes) {
-    p252_fr tag;
-    int rc = p252_hash_tag(merkle_domain(arity), (size_t)arity, 1, &tag);
-    if (rc != P252_OK) return rc;
-    const p252_fr* src = leaves;
-    p252_fr* dst = nodes;
-    for (size_t m = n_leaves / arity; m >= 1; m /= arity) {
-        cudaError_t le = p252::launch_digest(limbs(&tag), src, m, (uint32_t)arity, dst, 1, false, ctx->coop_max, ctx->stream);
-        if (le != cudaSuccess) return fail_cuda(ctx, le, "kernel launch");
-        ctx->launches++;
-        src = dst;
-        dst += m;
-        if (m == 1) break;
+// Heights from+1 .. depth, one launch each, reading height `from` where t.level(leaves, nodes, from) points.
+static int merkle_build_levels(p252_ctx* ctx, const Tree& t, const p252_fr* leaves, p252_fr* nodes, int from) {
+    for (int h = from + 1; h <= t.depth; ++h) {
+        int rc = count_launch(ctx, p252::launch_digest(limbs(&t.tag), t.level<const p252_fr>(leaves, nodes, h - 1), t.size(h),
+                                                       (uint32_t)t.arity, nodes + t.offset(h), 1, false, ctx->coop_max,
+                                                       ctx->stream));
+        if (rc != P252_OK) return rc;
     }
     return P252_OK;
 }
 
 int p252_merkle_build(p252_ctx* ctx, int arity, const p252_fr* leaves, size_t n_leaves, p252_fr* nodes_out, int flags) {
     if (!ctx || !leaves || !nodes_out) return P252_ERR_INVALID_ARGUMENT;
-    size_t n_internal;
-    int rc = p252_merkle_tree_nodes(arity, n_leaves, &n_internal, nullptr);
+    Tree t;
+    int rc = make_tree(arity, n_leaves, &t);
     if (rc != P252_OK) return rc;
     P252_LOCK(ctx);
     DeviceGuard g(ctx->device);
     if (flags & P252_MEM_DEVICE) {
         if (!aligned16(leaves) || !aligned16(nodes_out)) return P252_ERR_INVALID_ARGUMENT;
-        rc = merkle_build_device(ctx, arity, leaves, n_leaves, nodes_out);
-        if (rc != P252_OK) return rc;
-        if (!(flags & P252_ASYNC)) CU(cudaStreamSynchronize(ctx->stream));
-        return P252_OK;
+        return device_call(ctx, flags, nullptr, [&](auto) { return merkle_build_levels(ctx, t, leaves, nodes_out, 0); });
     }
-    // HOST: the first (largest) level streams through the chunked pipeline straight from the host
-    // leaves; the remaining levels run on the device-resident level.
-    const size_t first = n_leaves / arity;
+    // HOST: height 1 (the largest level) streams through the chunked pipeline straight from the host leaves; the
+    // heights above run on the device-resident internal nodes.
+    const size_t first = t.size(1);
     p252_fr* d_nodes = nullptr;
-    CU(cudaMalloc(reinterpret_cast<void**>(&d_nodes), n_internal * sizeof(p252_fr)));
-    p252_fr tag;
-    p252_hash_tag(merkle_domain(arity), (size_t)arity, 1, &tag);
+    CU(cudaMalloc(reinterpret_cast<void**>(&d_nodes), t.n_internal * sizeof(p252_fr)));
     {
         std::vector<Io> ios = {{leaves, nullptr, (size_t)arity * 32}, {nullptr, nodes_out, 32}};
         size_t done = 0;   // the pipeline hands chunks in order; mirror each chunk into d_nodes as well
         rc = run_host_pipeline(ctx, ios, first, [&](void** d, size_t cnt, cudaStream_t st) {
-            cudaError_t e = p252::launch_digest(limbs(&tag), d[0], cnt, (uint32_t)arity, d[1], 1, false, ctx->coop_max, st);
+            cudaError_t e = p252::launch_digest(limbs(&t.tag), d[0], cnt, (uint32_t)arity, d[1], 1, false, ctx->coop_max, st);
             if (e != cudaSuccess) return e;
             e = cudaMemcpyAsync(d_nodes + done, d[1], cnt * sizeof(p252_fr), cudaMemcpyDeviceToDevice, st);
             done += cnt;
             return e;
         });
     }
-    if (rc == P252_OK && first > 1) {
-        rc = merkle_build_device(ctx, arity, d_nodes, first, d_nodes + first);
+    if (rc == P252_OK && t.depth > 1) {
+        rc = merkle_build_levels(ctx, t, nullptr, d_nodes, 1);
         if (rc == P252_OK) {
-            cudaError_t e = cudaMemcpyAsync(nodes_out + first, d_nodes + first, (n_internal - first) * sizeof(p252_fr),
+            cudaError_t e = cudaMemcpyAsync(nodes_out + first, d_nodes + first, (t.n_internal - first) * sizeof(p252_fr),
                                             cudaMemcpyDeviceToHost, ctx->stream);
             if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
             if (e != cudaSuccess) rc = fail_cuda(ctx, e, "merkle D2H");
@@ -798,19 +825,11 @@ int p252_merkle4_build(p252_ctx* ctx, const p252_fr* leaves, size_t n_leaves, p2
 }
 
 // ---- Merkle openings ----------------------------------------------------------------------------------------
-static int tree_depth(int arity, size_t n_leaves, int* depth) {
-    int lv = 0;
-    int rc = p252_merkle_tree_nodes(arity, n_leaves, nullptr, &lv);
-    if (rc != P252_OK) return rc;
-    *depth = lv;
-    return P252_OK;
-}
-
 int p252_merkle_open_batch(p252_ctx* ctx, int arity, const p252_fr* leaves, size_t n_leaves, const p252_fr* nodes,
                            const uint64_t* leaf_idx, size_t n, p252_fr* paths_out, int flags) {
     if (!ctx || !leaves || !nodes || ((!leaf_idx || !paths_out) && n)) return P252_ERR_INVALID_ARGUMENT;
-    int depth = 0;
-    int rc = tree_depth(arity, n_leaves, &depth);
+    Tree t;
+    int rc = make_tree(arity, n_leaves, &t);
     if (rc != P252_OK) return rc;
     P252_LOCK(ctx);
     DeviceGuard g(ctx->device);
@@ -818,29 +837,21 @@ int p252_merkle_open_batch(p252_ctx* ctx, int arity, const p252_fr* leaves, size
         if (!aligned16(leaves) || !aligned16(nodes) || !aligned16(paths_out) || (reinterpret_cast<uintptr_t>(leaf_idx) & 7))
             return P252_ERR_INVALID_ARGUMENT;
         if (n == 0) return P252_OK;
-        return finish_device_call(ctx, p252::launch_merkle_open(leaves, nodes, leaf_idx, n, arity, (uint32_t)depth,
-                                                                n_leaves, paths_out, ctx->stream), flags);
+        return device_call(ctx, flags, nullptr, [&](auto) {
+            return count_launch(ctx, p252::launch_merkle_open(leaves, nodes, leaf_idx, n, arity, (uint32_t)t.depth, n_leaves,
+                                                              paths_out, ctx->stream));
+        });
     }
     // HOST tree: an opening is a pure gather of 32-byte items the caller already holds in host memory -- shipping
     // the whole tree to the GPU to copy depth*arity scalars back would only add PCIe traffic.  No hashing happens here.
-    std::vector<size_t> off((size_t)depth, 0);       // offset of internal level l-1 inside nodes, for l >= 1
-    {
-        size_t m = n_leaves / (size_t)arity, acc = 0;
-        for (int l = 1; l < depth; ++l, m /= (size_t)arity) {
-            off[(size_t)l] = acc;
-            acc += m;
-        }
-    }
     for (size_t i = 0; i < n; ++i)
         if (leaf_idx[i] >= n_leaves) return P252_ERR_INVALID_ARGUMENT;
     const size_t A = (size_t)arity;
     for (size_t i = 0; i < n; ++i) {
-        uint64_t idx = leaf_idx[i];
-        for (int l = 0; l < depth; ++l) {
-            const uint64_t group = idx / A;
-            const p252_fr* src = (l == 0) ? leaves + group * A : nodes + off[(size_t)l] + group * A;
-            memcpy(paths_out + (i * (size_t)depth + (size_t)l) * A, src, A * sizeof(p252_fr));
-            idx = group;
+        uint64_t grp = leaf_idx[i];
+        for (int h = 0; h < t.depth; ++h) {
+            grp >>= t.log2_arity;   // the group of the path node at height h
+            memcpy(paths_out + (i * (size_t)t.depth + (size_t)h) * A, t.group(leaves, nodes, h, grp), A * sizeof(p252_fr));
         }
     }
     return P252_OK;
@@ -850,9 +861,9 @@ int p252_merkle_verify_batch(p252_ctx* ctx, int arity, int depth, const p252_fr*
                              const p252_fr* paths, const p252_fr* root, size_t n, uint8_t* ok, size_t* n_failed,
                              int flags) {
     if (!ctx || !root || ((!leaf_items || !leaf_idx || !paths || !ok) && n)) return P252_ERR_INVALID_ARGUMENT;
-    if (merkle_domain(arity) < 0 || depth < 1 || depth > 64) return P252_ERR_INVALID_ARGUMENT;
+    if (depth < 1 || depth > p252::kMaxDepth) return P252_ERR_INVALID_ARGUMENT;
     p252_fr tag;
-    int rc = p252_hash_tag(merkle_domain(arity), (size_t)arity, 1, &tag);
+    int rc = merkle_tag(arity, &tag);
     if (rc != P252_OK) return rc;
     P252_LOCK(ctx);
     DeviceGuard g(ctx->device);
@@ -861,14 +872,10 @@ int p252_merkle_verify_batch(p252_ctx* ctx, int arity, int depth, const p252_fr*
         if (!aligned16(leaf_items) || !aligned16(paths) || (reinterpret_cast<uintptr_t>(leaf_idx) & 7))
             return P252_ERR_INVALID_ARGUMENT;
         if (n == 0) return P252_OK;
-        if (n_failed && (rc = counter_begin(ctx)) != P252_OK) return rc;
-        cudaError_t le = p252::launch_merkle_verify(limbs(&tag), limbs(root), leaf_items, leaf_idx, paths, n, arity,
-                                                    (uint32_t)depth, ok, n_failed ? ctx->d_counter : nullptr, ctx->stream);
-        if (le != cudaSuccess) return fail_cuda(ctx, le, "kernel launch");
-        ctx->launches++;
-        if ((rc = counter_end(ctx, n_failed)) != P252_OK) return rc;
-        if (!(flags & P252_ASYNC)) CU(cudaStreamSynchronize(ctx->stream));
-        return P252_OK;
+        return device_call(ctx, flags, n_failed, [&](unsigned long long* failed) {
+            return count_launch(ctx, p252::launch_merkle_verify(limbs(&tag), limbs(root), leaf_items, leaf_idx, paths, n, arity,
+                                                                (uint32_t)depth, ok, failed, ctx->stream));
+        });
     }
     const size_t path_bytes = (size_t)depth * (size_t)arity * 32;
     std::vector<Io> ios = {{leaf_items, nullptr, 32}, {leaf_idx, nullptr, 8}, {paths, nullptr, path_bytes}, {nullptr, ok, 1}};
@@ -876,12 +883,7 @@ int p252_merkle_verify_batch(p252_ctx* ctx, int arity, int depth, const p252_fr*
         return p252::launch_merkle_verify(limbs(&tag), limbs(root), d[0], static_cast<const uint64_t*>(d[1]), d[2], cnt, arity,
                                           (uint32_t)depth, static_cast<uint8_t*>(d[3]), nullptr, st);
     });
-    if (rc == P252_OK && n_failed) {
-        size_t bad = 0;
-        for (size_t i = 0; i < n; ++i) bad += ok[i] ? 0 : 1;
-        *n_failed = bad;
-    }
-    return rc;
+    return count_failed(rc, ok, n, n_failed);
 }
 
 // ---- incremental Merkle updates ---------------------------------------------------------------------------------
@@ -904,42 +906,35 @@ static int update_scratch(p252_ctx* ctx, size_t bytes, void** out) {
 
 // DEVICE: everything is enqueued on the context stream -- planning (p252::launch_merkle_update_plan) and then one
 // hash launch per level, sized by min(k, level size); each kernel reads its level's real list length on the device.
-static int merkle_update_device(p252_ctx* ctx, int arity, int depth, const p252_fr* tag, p252_fr* leaves, size_t n_leaves,
-                                p252_fr* nodes, const uint64_t* leaf_idx, const p252_fr* values, size_t k,
-                                size_t* n_rejected) {
-    const int s = arity == 4 ? 2 : 1;
-    p252::MerkleUpdatePlan plan = p252::merkle_update_layout(nullptr, k, s, (uint32_t)depth, n_leaves);
+static int merkle_update_device(p252_ctx* ctx, const Tree& t, p252_fr* leaves, p252_fr* nodes, const uint64_t* leaf_idx,
+                                const p252_fr* values, size_t k, size_t* n_rejected, int flags) {
+    const uint32_t depth = (uint32_t)t.depth;
+    p252::MerkleUpdatePlan plan = p252::merkle_update_layout(nullptr, k, t.log2_arity, depth, t.n_leaves);
     void* scratch = nullptr;
     int rc = update_scratch(ctx, plan.total_bytes, &scratch);
     if (rc != P252_OK) return rc;
-    plan = p252::merkle_update_layout(scratch, k, s, (uint32_t)depth, n_leaves);
-    if (n_rejected && (rc = counter_begin(ctx)) != P252_OK) return rc;
-    cudaError_t le = p252::launch_merkle_update_plan(plan, leaf_idx, values, k, s, (uint32_t)depth, n_leaves, leaves,
-                                                     n_rejected ? ctx->d_counter : nullptr, ctx->stream);
-    if (le != cudaSuccess) return fail_cuda(ctx, le, "merkle update plan");
-    ctx->launches += 2;
-    const p252_fr* below = leaves;
-    p252_fr* level = nodes;
-    for (int l = 0; l < depth; ++l) {
-        const size_t m = n_leaves >> (s * (l + 1));   // nodes of level l + 1
-        le = p252::launch_merkle_update(limbs(tag), arity, below, plan.lists[l], plan.lists[l], level, std::min(k, m),
-                                        plan.counts + l, m, ctx->coop_max, ctx->stream);
-        if (le != cudaSuccess) return fail_cuda(ctx, le, "kernel launch");
-        ctx->launches++;
-        below = level;
-        level += m;
-    }
-    return counter_end(ctx, n_rejected);
+    plan = p252::merkle_update_layout(scratch, k, t.log2_arity, depth, t.n_leaves);
+    return device_call(ctx, flags, n_rejected, [&](unsigned long long* rejected) {
+        int st = count_launch(ctx, p252::launch_merkle_update_plan(plan, leaf_idx, values, k, t.log2_arity, depth, t.n_leaves,
+                                                                   leaves, rejected, ctx->stream),
+                              "merkle update plan", 2);
+        for (int h = 1; h <= t.depth && st == P252_OK; ++h)   // plan.lists[h - 1]: the dirty nodes of height h
+            st = count_launch(ctx, p252::launch_merkle_update(limbs(&t.tag), t.arity, t.level(leaves, nodes, h - 1),
+                                                              plan.lists[h - 1], plan.lists[h - 1], t.level(leaves, nodes, h),
+                                                              std::min(k, t.size(h)), plan.counts + h - 1, t.size(h),
+                                                              ctx->coop_max, ctx->stream));
+        return st;
+    });
 }
 
 // HOST: only the dirty paths travel.  The children groups of every dirty parent are staged with one H2D (level 1:
 // leaves with the new values applied; above: the current nodes, whose dirty entries the level below overwrites on the
 // device), every level's kernel writes its parents into their slots among the next level's staged groups (the top
 // level into a one-slot buffer), one D2H brings the groups back, and only then are the caller's arrays written.
-static int merkle_update_host(p252_ctx* ctx, int arity, int depth, const p252_fr* tag, p252_fr* leaves, size_t n_leaves,
-                              p252_fr* nodes, const uint64_t* leaf_idx, const p252_fr* values, size_t k) {
-    const int s = arity == 4 ? 2 : 1;
-    const size_t A = (size_t)arity;
+static int merkle_update_host(p252_ctx* ctx, const Tree& t, p252_fr* leaves, p252_fr* nodes, const uint64_t* leaf_idx,
+                              const p252_fr* values, size_t k) {
+    const int depth = t.depth, s = t.log2_arity;
+    const size_t A = (size_t)t.arity;
     // dedupe: stable order by index, the last occurrence of an index wins
     std::vector<uint32_t> ord(k);
     for (size_t i = 0; i < k; ++i) ord[i] = (uint32_t)i;
@@ -964,12 +959,10 @@ static int merkle_update_host(p252_ctx* ctx, int arity, int depth, const p252_fr
     const size_t stage_bytes = n_stage * sizeof(p252_fr);
     std::vector<p252_fr> stage(n_stage);
     std::vector<uint64_t> widx(n_widx);
-    std::vector<size_t> off((size_t)depth + 1, 0);   // offset of internal level l inside nodes
-    for (int l = 2; l <= depth; ++l) off[(size_t)l] = off[(size_t)l - 1] + (n_leaves >> (s * (l - 1)));
     for (int l = 1; l <= depth; ++l) {
         const std::vector<uint64_t>& L = list[(size_t)l];
-        const p252_fr* src = (l == 1) ? leaves : nodes + off[(size_t)l - 1];
-        for (size_t j = 0; j < L.size(); ++j) memcpy(&stage[region[(size_t)l] + j * A], src + L[j] * A, A * sizeof(p252_fr));
+        for (size_t j = 0; j < L.size(); ++j)
+            memcpy(&stage[region[(size_t)l] + j * A], t.group(leaves, nodes, l - 1, L[j]), A * sizeof(p252_fr));
         if (l == depth) {
             widx[widx_off[(size_t)l]] = 0;
             continue;
@@ -998,11 +991,10 @@ static int merkle_update_host(p252_ctx* ctx, int arity, int depth, const p252_fr
         for (int l = 1; l <= depth; ++l) {
             const size_t n = list[(size_t)l].size();
             p252_fr* out = d_stage + region[(size_t)l + 1];   // the next level's groups, or the root slot
-            cudaError_t le = p252::launch_merkle_update(limbs(tag), arity, d_stage + region[(size_t)l], nullptr,
-                                                        d_widx + widx_off[(size_t)l], out, n, nullptr, n, ctx->coop_max,
-                                                        ctx->stream);
-            if (le != cudaSuccess) return fail_cuda(ctx, le, "kernel launch");
-            ctx->launches++;
+            int st = count_launch(ctx, p252::launch_merkle_update(limbs(&t.tag), t.arity, d_stage + region[(size_t)l], nullptr,
+                                                                  d_widx + widx_off[(size_t)l], out, n, nullptr, n,
+                                                                  ctx->coop_max, ctx->stream));
+            if (st != P252_OK) return st;
         }
         CU(cudaMemcpyAsync(stage.data() + region[2], d_stage + region[2], (n_stage - region[2]) * sizeof(p252_fr),
                            cudaMemcpyDeviceToHost, ctx->stream));
@@ -1019,9 +1011,9 @@ static int merkle_update_host(p252_ctx* ctx, int arity, int depth, const p252_fr
     for (int l = 1; l < depth; ++l) {
         const std::vector<uint64_t>& L = list[(size_t)l];
         for (size_t j = 0; j < L.size(); ++j)
-            nodes[off[(size_t)l] + L[j]] = stage[region[(size_t)l + 1] + widx[widx_off[(size_t)l] + j]];
+            t.level(leaves, nodes, l)[L[j]] = stage[region[(size_t)l + 1] + widx[widx_off[(size_t)l] + j]];
     }
-    nodes[off[(size_t)depth]] = stage[region[(size_t)depth + 1]];
+    *t.level(leaves, nodes, depth) = stage[region[(size_t)depth + 1]];
     for (uint32_t u : upd) leaves[leaf_idx[u]] = values[u];
     return P252_OK;
 }
@@ -1029,12 +1021,10 @@ static int merkle_update_host(p252_ctx* ctx, int arity, int depth, const p252_fr
 int p252_merkle_update_batch(p252_ctx* ctx, int arity, p252_fr* leaves, size_t n_leaves, p252_fr* nodes,
                              const uint64_t* leaf_idx, const p252_fr* values, size_t k, size_t* n_rejected, int flags) {
     if (!ctx || !leaves || !nodes || ((!leaf_idx || !values) && k)) return P252_ERR_INVALID_ARGUMENT;
-    int depth = 0;
-    int rc = tree_depth(arity, n_leaves, &depth);
+    Tree t;
+    int rc = make_tree(arity, n_leaves, &t);
     if (rc != P252_OK) return rc;
     if (k > 0xffffffffull) return P252_ERR_INVALID_ARGUMENT;   // batch positions are 32-bit
-    p252_fr tag;
-    if ((rc = p252_hash_tag(merkle_domain(arity), (size_t)arity, 1, &tag)) != P252_OK) return rc;
     P252_LOCK(ctx);
     DeviceGuard g(ctx->device);
     if (n_rejected) *n_rejected = 0;
@@ -1042,15 +1032,12 @@ int p252_merkle_update_batch(p252_ctx* ctx, int arity, p252_fr* leaves, size_t n
         if (!aligned16(leaves) || !aligned16(nodes) || !aligned16(values) || (reinterpret_cast<uintptr_t>(leaf_idx) & 7))
             return P252_ERR_INVALID_ARGUMENT;
         if (k == 0) return P252_OK;
-        rc = merkle_update_device(ctx, arity, depth, &tag, leaves, n_leaves, nodes, leaf_idx, values, k, n_rejected);
-        if (rc != P252_OK) return rc;
-        if (!(flags & P252_ASYNC)) CU(cudaStreamSynchronize(ctx->stream));
-        return P252_OK;
+        return merkle_update_device(ctx, t, leaves, nodes, leaf_idx, values, k, n_rejected, flags);
     }
     for (size_t i = 0; i < k; ++i)
         if (leaf_idx[i] >= n_leaves) return P252_ERR_INVALID_ARGUMENT;   // before anything is written
     if (k == 0) return P252_OK;
-    return merkle_update_host(ctx, arity, depth, &tag, leaves, n_leaves, nodes, leaf_idx, values, k);
+    return merkle_update_host(ctx, t, leaves, nodes, leaf_idx, values, k);
 }
 
 // ---- multi-GPU ------------------------------------------------------------------------------------------
@@ -1068,8 +1055,8 @@ int p252_dist_unique_id(uint8_t id[P252_NCCL_UNIQUE_ID_BYTES]) {
 
 int p252_dist_init(p252_ctx* ctx, const uint8_t id[P252_NCCL_UNIQUE_ID_BYTES], int rank, int nranks) {
     if (!ctx || !id || nranks < 1 || rank < 0 || rank >= nranks) return P252_ERR_INVALID_ARGUMENT;
-    if (ctx->comm) return P252_ERR_INVALID_ARGUMENT;
     P252_LOCK(ctx);
+    if (ctx->comm) return P252_ERR_INVALID_ARGUMENT;
     DeviceGuard g(ctx->device);
     if (!nccl().ok) return fail_nccl(ctx, ncclSystemError, "dlopen(libnccl.so.2)");
     ncclUniqueId u;
@@ -1107,23 +1094,21 @@ int p252_dist_finalize(p252_ctx* ctx) {
 int p252_merkle4_shard_plan(size_t n_leaves_total, int nranks, int rank, p252_level_plan* levels, int capacity,
                             int* n_levels) {
     if (nranks < 1 || rank < 0 || rank >= nranks) return P252_ERR_INVALID_ARGUMENT;
-    int lv = 0;
-    int rc = p252_merkle4_tree_nodes(n_leaves_total, nullptr, &lv);
+    Tree t;
+    int rc = make_tree(4, n_leaves_total, &t);
     if (rc != P252_OK) return rc;
     if (n_leaves_total % (size_t)nranks || (n_leaves_total / nranks) % 4) return P252_ERR_INVALID_ARGUMENT;
-    if (n_levels) *n_levels = lv;
+    if (n_levels) *n_levels = t.depth;
     if (!levels) return P252_OK;
-    if (capacity < lv) return P252_ERR_INVALID_ARGUMENT;
-    uint64_t off = 0, m = n_leaves_total / 4;
-    for (int l = 0; l < lv; ++l, m /= 4) {
-        p252_level_plan& p = levels[l];
-        p.level_offset = off;
-        p.level_size = m;
-        p.sharded = (m % (uint64_t)nranks == 0) ? 1 : 0;
-        p.my_count = p.sharded ? m / nranks : m;
+    if (capacity < t.depth) return P252_ERR_INVALID_ARGUMENT;
+    for (int h = 1; h <= t.depth; ++h) {
+        p252_level_plan& p = levels[h - 1];
+        p.level_offset = t.offset(h);
+        p.level_size = t.size(h);
+        p.sharded = (p.level_size % (uint64_t)nranks == 0) ? 1 : 0;
+        p.my_count = p.sharded ? p.level_size / nranks : p.level_size;
         p.my_offset = p.sharded ? (uint64_t)rank * p.my_count : 0;
         p.reserved = 0;
-        off += m;
     }
     return P252_OK;
 }
@@ -1133,16 +1118,16 @@ int p252_merkle4_build_dist(p252_ctx* ctx, const p252_fr* leaves_shard, size_t n
     if (!ctx || !leaves_shard || !nodes_out) return P252_ERR_INVALID_ARGUMENT;
     if (!(flags & P252_MEM_DEVICE)) return P252_ERR_INVALID_ARGUMENT;   // shards live on the GPU
     if (!aligned16(leaves_shard) || !aligned16(nodes_out)) return P252_ERR_INVALID_ARGUMENT;
+    P252_LOCK(ctx);
     const int G = ctx->nranks, r = ctx->rank;
     if (G > 1 && !ctx->comm) return P252_ERR_INVALID_ARGUMENT;
-    p252_level_plan plan[64];
+    p252_level_plan plan[p252::kMaxDepth];
     int lv = 0;
-    int rc = p252_merkle4_shard_plan(n_leaves_total, G, r, plan, 64, &lv);
+    int rc = p252_merkle4_shard_plan(n_leaves_total, G, r, plan, p252::kMaxDepth, &lv);
     if (rc != P252_OK) return rc;
-    P252_LOCK(ctx);
-    DeviceGuard g(ctx->device);
     p252_fr tag;
-    p252_hash_tag(P252_DOMAIN_MERKLE4, 4, 1, &tag);
+    if ((rc = merkle_tag(4, &tag)) != P252_OK) return rc;
+    DeviceGuard g(ctx->device);
 
     const bool timing = (flags & P252_TIMING) != 0;
     const bool no_gather = (flags & P252_NO_GATHER) != 0;
@@ -1172,9 +1157,9 @@ int p252_merkle4_build_dist(p252_ctx* ctx, const p252_fr* leaves_shard, size_t n
         if (p.sharded) {
             // the first level is always sharded (n_leaves_total / G is a multiple of 4)
             if (timing) CU(cudaEventRecord(ctx->level_events[(size_t)l].k0, ctx->stream));
-            cudaError_t le = p252::launch_digest(limbs(&tag), below_mine, p.my_count, 4, level + p.my_offset, 1, false, ctx->coop_max, ctx->stream);
-            if (le != cudaSuccess) return fail_cuda(ctx, le, "kernel launch");
-            ctx->launches++;
+            rc = count_launch(ctx, p252::launch_digest(limbs(&tag), below_mine, p.my_count, 4, level + p.my_offset, 1, false,
+                                                       ctx->coop_max, ctx->stream));
+            if (rc != P252_OK) return rc;
             if (timing) CU(cudaEventRecord(ctx->level_events[(size_t)l].k1, ctx->stream));
             if (G > 1 && !no_gather) {
                 CU(cudaEventRecord(ctx->ev_level, ctx->stream));
@@ -1196,9 +1181,9 @@ int p252_merkle4_build_dist(p252_ctx* ctx, const p252_fr* leaves_shard, size_t n
                 gather_in_flight = false;
             }
             if (timing) CU(cudaEventRecord(ctx->level_events[(size_t)l].k0, ctx->stream));
-            cudaError_t le = p252::launch_digest(limbs(&tag), below_full, p.level_size, 4, level, 1, false, ctx->coop_max, ctx->stream);
-            if (le != cudaSuccess) return fail_cuda(ctx, le, "kernel launch");
-            ctx->launches++;
+            rc = count_launch(ctx, p252::launch_digest(limbs(&tag), below_full, p.level_size, 4, level, 1, false, ctx->coop_max,
+                                                       ctx->stream));
+            if (rc != P252_OK) return rc;
             if (timing) CU(cudaEventRecord(ctx->level_events[(size_t)l].k1, ctx->stream));
         }
         below_full = level;
